@@ -2,6 +2,7 @@
 """Benchmark of the NeuralRecon-W per-ray training hot path on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl nrw|reference] [--precision bf16x3|bf16|bf16x6]
+                    [--dump-outputs DIR]
 
 A "step" = one full training step over one batch of 8192 synthetic posed-camera rays x 128 samples
 (BASELINE config C2 "brandenburg_gate config, 8192 rays x 128 samples"): voxel-guided hierarchical
@@ -137,6 +138,19 @@ def peaks():
         d = json.load(open(p))
         return d.get("bf16_tflops_sustained", 1409.5), d.get("hbm_gbs", 6576.7), "measured (MEASURED_PEAKS.json, sustained bf16)"
     return 1400.0, 6650.0, "fallback (B200_PROFILING.md)"
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: what the last timed step computed, as out_dir/<name>.npy (float32), so that two builds run with the
+    same arguments (hence the same seeded inputs) can be compared output for output."""
+    import numpy as np
+
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.detach().float().cpu().numpy())
+
+
+DUMP_SAMPLE = 1 << 22      # C5 volume entries written by --dump-outputs (16 MB of the 512 MB volume, a fixed seeded sample)
 
 
 # ----------------------------------------------------------------------------------------------
@@ -322,6 +336,9 @@ def bench_c5(args, rank, world, local):
     l0 = L.nrw_launch_count()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier(); e0.record(); vol = run(args.steps, False); e1.record(); barrier()
+    if args.dump_outputs and rank == 0:
+        idx = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+        dump_outputs(args.dump_outputs, {"sdf_volume_sample": vol.reshape(-1)[idx.to(device)]})
     launches = (L.nrw_launch_count() - l0) // max(args.steps, 1)
     ms = e0.elapsed_time(e1) / args.steps
     clk = clocks.stop() if rank == 0 else None
@@ -401,6 +418,8 @@ def main():
     ap.add_argument("--no_cpu_baseline", action="store_true")
     ap.add_argument("--no_torch_gpu_ref", action="store_true")
     ap.add_argument("--no_other_modes", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (float32, < 64 MB in all)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
@@ -505,6 +524,10 @@ def main():
     warm = max(args.warmup, 3)
     run(warm, False)
     ms, clk, launches, loss = timed(args.steps, False)
+    if args.dump_outputs and rank == 0:     # the step's loss, the parameters it updated and the gradient it applied
+        eng = sysm.renderer.engine
+        dump_outputs(args.dump_outputs, {"loss": loss.reshape(1), "params_flat": eng.flat, "grad_flat": eng.last_flat_grad,
+                                         "embedding_a": sysm.embedding_a.weight})
     run(1, True)
     ms_e2e, clk2, _, _ = timed(args.steps, True)
     t = torch.tensor([ms, ms_e2e], device=device, dtype=torch.float64)

@@ -122,6 +122,159 @@ def grad_probe(grads, n_probe=4, seed=99):
     return out
 
 
+def sample_index(numel, key, n=256):
+    """Seeded, sorted sample of up to n flat indices of a tensor with `numel` elements (depends on the name only)."""
+    gen = torch.Generator().manual_seed(7 + (sum(map(ord, key)) % 100003))
+    return torch.randperm(numel, generator=gen)[:n].sort().values
+
+
+# tests/test_dataio_oracle.py: (n_items, world) of DataModule._get_local_split, (n, world) of utils.visualization.get_local_split
+DATAIO_SPLITS = [(64, 8), (64, 3), (5, 4), (7, 1)]
+DATAIO_RANGES = [(10, 4), (12, 4), (1, 3)]
+
+
+def dataio_getitem_inputs():
+    """500 ray-cache rows (rays[12] with image id / semantic label columns, rgbs[3]) and 97 drawn indices."""
+    g = torch.Generator().manual_seed(0)
+    n = 500
+    all_rays = torch.randn(n, 12, generator=g)
+    all_rays[:, 8] = torch.randint(0, 1500, (n,), generator=g).float()
+    all_rays[:, 9] = torch.tensor([0.0, 2.0, 12.0, 20.0, 116.0, 127.0, 6.0])[torch.randint(0, 7, (n,), generator=g)]
+    all_rgbs = torch.rand(n, 3, generator=g)
+    idx = torch.randperm(n, generator=g)[:97]
+    return all_rays, all_rgbs, idx
+
+
+def make_dataio_golden():
+    """The reference's data-path helpers on the inputs of tests/test_dataio_oracle.py -> tests/golden/dataio.npz."""
+    ref_import.load()
+    from datasets.data import DataModule  # type: ignore
+    from datasets.mask_utils import get_label_id_mapping  # type: ignore
+    from datasets.phototourism import PhototourismDataset  # type: ignore
+    from utils.visualization import get_local_split  # type: ignore
+
+    arrays = {}
+    for n_items, world in DATAIO_SPLITS:
+        items = [f"split_{i}" for i in range(n_items)]
+        for rank in range(world):
+            want = DataModule._get_local_split(None, items, world, rank)
+            arrays[f"split.{n_items}_{world}_{rank}"] = np.array([int(s[len("split_"):]) for s in want], np.int64)
+    all_rays, all_rgbs, idx = dataio_getitem_inputs()
+    fake = types.SimpleNamespace(split="train", all_rays=all_rays, all_rgbs=all_rgbs, with_semantics=True)
+    items = [PhototourismDataset.__getitem__(fake, int(i)) for i in idx]
+    for k in items[0]:
+        arrays["getitem." + k] = torch.stack([it[k] for it in items]).numpy()
+    m = get_label_id_mapping()
+    arrays["label.names"] = np.array(sorted(m))
+    arrays["label.ids"] = np.array([m[k] for k in sorted(m)], np.int64)
+    for n, world in DATAIO_RANGES:
+        data = torch.arange(n * 3, dtype=torch.float32).reshape(n, 3) + 1
+        for rank in range(world):
+            arrays[f"local.{n}_{world}_{rank}"] = get_local_split(data, world, rank).numpy()
+    return arrays
+
+
+# tests/test_oracle_vs_reference.py: a config unlike the CASES below (s_val_base 2, cos_anneal 0.25, 6 outside samples)
+PORT_CFG = dict(n_samples=12, n_importance=12, up_sample_steps=3, n_outside=6, s_val_base=2, cos_anneal_ratio=0.25)
+PORT_RAYS, PORT_SEED = 24, 5
+
+
+def make_port_golden():
+    """One training step of the reference on the PORT_CFG batch (every output, the loss, a seeded sample of every parameter
+    gradient with its max magnitude) and the reference modules' state_dict layout -> tests/golden/port_step.npz."""
+    import json
+
+    P = synth.make_params(seed=0)
+    cfg = synth.PathConfig(**PORT_CFG, **synth.BRANDENBURG)
+    batch = synth.make_rays(PORT_RAYS, cfg, seed=PORT_SEED)
+    res, loss, grads, _ = reference_train_step(cfg, P, batch, perturb_overwrite=0)
+    arrays = {f"out.{k}": v.detach().numpy() for k, v in res.items()}
+    arrays["loss"] = loss.numpy()
+    for k, g in grads.items():
+        flat = g.reshape(-1)
+        arrays["gs." + k] = flat[sample_index(flat.numel(), k)].numpy()
+        arrays["gmax." + k] = flat.abs().max().numpy()
+    m = build_reference(synth.PathConfig(), P)
+    layout = {}
+    for pre, mod in (("neuconw.", m["neuconw"]), ("nerf.", m["nerf"]), ("embedding_a.", m["emb"])):
+        for k, v in mod.state_dict().items():
+            layout[pre + k] = list(v.shape)
+    arrays["state_dict_layout"] = np.array(json.dumps(layout, sort_keys=True))
+    return arrays
+
+
+# tests/test_gpu_fullsize_reference.py: the full C2 batch is stored for a seeded sample of its rays
+FULL_RAYS, FULL_SEED, FULL_SAMPLE_RAYS, FULL_SAMPLE_GRAD = 8192, 17, 128, 32768
+FULL_PER_RAY = ("color", "color_sphere", "color_bg", "cdf_fine", "gradients", "mask_error", "weights", "weights_sum", "weights_max",
+                "inside_sphere", "depth")
+
+
+def full_sample():
+    """(ray indices, flat-gradient indices over the sorted neuconw. / nerf. parameter names) of the stored C2 sample."""
+    gen = torch.Generator().manual_seed(2024)
+    rays = torch.randperm(FULL_RAYS, generator=gen)[:FULL_SAMPLE_RAYS].sort().values
+    total = sum(v.numel() for k, v in synth.make_params(seed=0).items() if not k.startswith("embedding_a."))
+    return rays, torch.randperm(total, generator=gen)[:FULL_SAMPLE_GRAD].sort().values
+
+
+def flat_grad(grads):
+    return torch.cat([grads[k].double().reshape(-1) for k in sorted(grads)])
+
+
+def make_fullsize_golden(device):
+    """The reference's full training step on the whole C2 batch (8192 rays x 128 samples, fp32, TF32 off) on `device`:
+    the per-ray outputs and z_vals of FULL_SAMPLE_RAYS rays, the loss, gradient_error, the squared norm of the neuconw +
+    nerf gradient and FULL_SAMPLE_GRAD of its entries -> tests/golden/fullsize_c2.npz."""
+    cfg = synth.PathConfig(**synth.BRANDENBURG)
+    P = synth.make_params(seed=0)
+    b = {k: v.to(device) for k, v in synth.make_rays(FULL_RAYS, cfg, seed=FULL_SEED).items()}
+    torch.backends.cuda.matmul.allow_tf32 = False
+    m = build_reference(cfg, P)
+    for k in ("neuconw", "nerf", "emb"):
+        m[k].to(device)
+    with warnings.catch_warnings():
+        warnings.simplefilter("ignore")
+        res = m["renderer"].render(b["rays"], b["ts"], b["label"], perturb_overwrite=0,
+                                   background_rgb=torch.zeros([1, 3], device=device), cos_anneal_ratio=cfg.cos_anneal_ratio)
+        loss = sum(m["loss"](res, b["rgbs"]).values())
+        loss.backward()
+    o = ((b["rays"][:, 0:3] - m["renderer"].origin).float() / cfg.radius).float()       # render()'s own normalisation
+    with torch.no_grad():
+        _, z, _, _ = m["renderer"].sparse_sampler(o, b["rays"][:, 3:6], (b["rays"][:, 6:7] / cfg.radius).float(),
+                                                  (b["rays"][:, 7:8] / cfg.radius).float(), 0)
+    grads = {}
+    for pre, mod in (("neuconw.", m["neuconw"]), ("nerf.", m["nerf"])):
+        for k, p in mod.named_parameters():
+            grads[pre + k] = (p.grad if p.grad is not None else torch.zeros_like(p)).detach().cpu()
+    rays, gidx = full_sample()
+    g = flat_grad(grads)
+    arrays = {f"out.{k}": res[k].detach().cpu()[rays].numpy() for k in FULL_PER_RAY}
+    arrays.update(z_vals=z.cpu()[rays].numpy(), loss=loss.detach().cpu().numpy(),
+                  gradient_error=res["gradient_error"].detach().cpu().numpy(),
+                  grad_norm2=np.array(float((g * g).sum())), grad_sample=g[gidx].numpy())
+    return arrays
+
+
+def make_precision_golden(device):
+    """The reference's 300-step fp32 training run of tests/test_gpu_precision_policy.py on `device` (same initial
+    weights, batches and schedule): loss / PSNR / eikonal / s_val of every step -> tests/golden/precision_curve.npz."""
+    sys.path.insert(0, os.path.dirname(GOLDEN_DIR))
+    import test_gpu_precision_policy as tp  # type: ignore
+    from . import ref_runner
+
+    all_b = tp._scene_batches(17)
+    batches = [{k: v.to(device) for k, v in b.items()} for b in all_b[:16]]
+    init = tp._initial_weights()
+    cfg = tp._ref_cfg()
+    r = ref_runner.RefRunner(cfg, init, device=device, lr=tp.LR)
+    hist = []
+    for i in range(tp.STEPS):
+        cfg.cos_anneal_ratio = min(1.0, i / 50000)                    # NeuconWSystem.get_cos_anneal_ratio
+        r.train_step(batches[i % len(batches)], perturb_overwrite=0)
+        hist.append(torch.stack([r.last_metrics[k].reshape(()) for k in ("loss", "psnr", "eikonal", "s_val")]))
+    return {"curve": torch.stack(hist).cpu().numpy()}
+
+
 CASES = {
     # name: (cfg, n_rays, perturb_overwrite, torch seed for perturb draws)
     "small_det": (synth.PathConfig(n_samples=16, n_importance=8, up_sample_steps=2, n_outside=4), 48, 0, None),
@@ -136,11 +289,30 @@ CASES = {
 FINE_CASES = {"fine_c3"}
 
 
+def save(out_dir, name, arrays):
+    path = os.path.join(out_dir, f"{name}.npz")
+    np.savez_compressed(path, **arrays)
+    print(f"wrote {path}: {os.path.getsize(path) / 1024:.1f} KiB")
+
+
 def main():
+    """python -m oracle.make_golden [--cases] [--cpu-extra] [--gpu OUT_DIR]: no flag regenerates the CASES files; the
+    GPU files are written to OUT_DIR (then copied to tests/golden)."""
     if not ref_import.available():
         print("reference tree not available; cannot regenerate golden vectors", file=sys.stderr)
         sys.exit(1)
     os.makedirs(GOLDEN_DIR, exist_ok=True)
+    argv = sys.argv[1:] or ["--cases"]
+    if "--cpu-extra" in argv:
+        save(GOLDEN_DIR, "dataio", make_dataio_golden())
+        save(GOLDEN_DIR, "port_step", make_port_golden())
+    if "--gpu" in argv:
+        out = argv[argv.index("--gpu") + 1]
+        os.makedirs(out, exist_ok=True)
+        save(out, "fullsize_c2", make_fullsize_golden(torch.device("cuda", 0)))
+        save(out, "precision_curve", make_precision_golden(torch.device("cuda", 0)))
+    if "--cases" not in argv:
+        return
     P = synth.make_params(seed=0)
     for name, (cfg, n_rays, pov, rseed) in CASES.items():
         batch = synth.make_rays(n_rays, cfg, seed=11)

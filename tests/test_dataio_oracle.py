@@ -1,47 +1,38 @@
-"""CPU: pins oracle/dataio_port.py to the unmodified reference (where importable) and checks the host-side logic of
-nrw.raycache / nrw.mesh that needs no GPU."""
-import types
+"""CPU: pins oracle/dataio_port.py to the unmodified reference (its outputs on these inputs are stored in
+tests/golden/dataio.npz by oracle/make_golden.py) and checks the host-side logic of nrw.raycache / nrw.mesh that needs
+no GPU."""
+import os
 
 import numpy as np
 import pytest
 import torch
 
+from conftest import GOLDEN
 from oracle import dataio_port as dp
-from oracle import ref_import
-
-needs_ref = pytest.mark.skipif(not ref_import.available(), reason="reference tree not present")
+from oracle.make_golden import DATAIO_RANGES, DATAIO_SPLITS, dataio_getitem_inputs
 
 
-@needs_ref
-@pytest.mark.parametrize("n_items,world", [(64, 8), (64, 3), (5, 4), (7, 1)])
-def test_local_split_matches_reference(n_items, world):
-    ref_import.load()
-    from datasets.data import DataModule  # type: ignore
+@pytest.fixture(scope="module")
+def G():
+    return np.load(os.path.join(GOLDEN, "dataio.npz"))
+
+
+@pytest.mark.parametrize("n_items,world", DATAIO_SPLITS)
+def test_local_split_matches_reference(n_items, world, G):
     from nrw.raycache import local_split
 
     items = [f"split_{i}" for i in range(n_items)]
     for rank in range(world):
-        want = list(DataModule._get_local_split(None, items, world, rank))
+        want = [f"split_{i}" for i in G[f"split.{n_items}_{world}_{rank}"]]      # DataModule._get_local_split
         assert list(dp.local_split(items, world, rank)) == want
         assert local_split(items, world, rank) == want
 
 
-@needs_ref
-def test_getitem_and_filter_match_reference():
-    ref_import.load()
-    from datasets.phototourism import PhototourismDataset  # type: ignore
-
-    g = torch.Generator().manual_seed(0)
-    n = 500
-    all_rays = torch.randn(n, 12, generator=g)
-    all_rays[:, 8] = torch.randint(0, 1500, (n,), generator=g).float()
-    all_rays[:, 9] = torch.tensor([0.0, 2.0, 12.0, 20.0, 116.0, 127.0, 6.0])[torch.randint(0, 7, (n,), generator=g)]
-    all_rgbs = torch.rand(n, 3, generator=g)
-    fake = types.SimpleNamespace(split="train", all_rays=all_rays, all_rgbs=all_rgbs, with_semantics=True)
-    idx = torch.randperm(n, generator=g)[:97]
-    items = [PhototourismDataset.__getitem__(fake, int(i)) for i in idx]
-    collated = {k: torch.stack([it[k] for it in items]) for k in items[0]}
+def test_getitem_and_filter_match_reference(G):
+    all_rays, all_rgbs, idx = dataio_getitem_inputs()
+    collated = {k[len("getitem."):]: torch.from_numpy(G[k]) for k in G.files if k.startswith("getitem.")}   # PhototourismDataset.__getitem__
     got = dp.getitem_batch(all_rays, all_rgbs, idx)
+    assert set(got) == set(collated)
     for k in collated:
         assert torch.equal(collated[k], got[k]), k
     assert got["rays"].shape == (97, 10) and got["ts"].dtype == torch.int64
@@ -54,26 +45,19 @@ def test_getitem_and_filter_match_reference():
     assert 0 < f["rays"].shape[0] < 97
 
 
-@needs_ref
-def test_label_ids_match_reference():
-    ref_import.load()
-    from datasets.mask_utils import get_label_id_mapping  # type: ignore
-
-    m = get_label_id_mapping()
+def test_label_ids_match_reference(G):
+    m = dict(zip(G["label.names"].tolist(), G["label.ids"].tolist()))           # datasets.mask_utils.get_label_id_mapping
     for k, v in dp.LABEL_IDS.items():
         assert m[k] == v, k
 
 
-@needs_ref
-@pytest.mark.parametrize("n,world", [(10, 4), (12, 4), (1, 3)])
-def test_local_range_matches_reference_get_local_split(n, world):
-    ref_import.load()
-    from utils.visualization import get_local_split  # type: ignore
+@pytest.mark.parametrize("n,world", DATAIO_RANGES)
+def test_local_range_matches_reference_get_local_split(n, world, G):
     from nrw.mesh import _local_range
 
     data = torch.arange(n * 3, dtype=torch.float32).reshape(n, 3) + 1
     for rank in range(world):
-        want = get_local_split(data, world, rank)
+        want = torch.from_numpy(G[f"local.{n}_{world}_{rank}"])                  # utils.visualization.get_local_split
         a, b, per = dp.local_range(n, world, rank)
         assert (a, b, per) == _local_range(n, world, rank)
         assert want.shape[0] == per

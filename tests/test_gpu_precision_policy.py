@@ -1,28 +1,33 @@
 """GPU: evidence for the precision policy (VERDICT r1 next-round #5).  north_star: ">= 4x the reference's single-GPU
 PyTorch renderer ... with matching PSNR / eikonal loss".
 
-Protocol.  One 300-step training run of the UNMODIFIED reference's fp32 torch path on this GPU (oracle/_ref; clip 0.99 +
-Adam(eps=1e-7), deterministic strata, a learnable synthetic scene) is the baseline; its weights are snapshotted at steps
-100 / 200 / 300.  The same run (same initial weights, same batches) is repeated in `bf16x3` (3 bf16 products per GEMM),
-`mixed` (3 products forward, plain-bf16 backward GEMMs) and `bf16` (one product everywhere).
+Protocol.  One 300-step training run of the reference's fp32 training step on this GPU (clip 0.99 + Adam(eps=1e-7),
+deterministic strata, a learnable synthetic scene) is the baseline; its weights are snapshotted at steps 100 / 200 / 300.
+The baseline runs the restatement oracle/neuconw_port.py (pinned to the unmodified reference by tests/test_oracle_golden.py),
+and its curve is held against tests/golden/precision_curve.npz, the same run of the unmodified reference on a B200
+(oracle/make_golden.py): first step within 1e-4, the first 25 steps within 1 %.  The same run (same initial weights,
+same batches) is repeated in `bf16x3` (3 bf16 products per GEMM), `mixed` (3 products forward, plain-bf16 backward
+GEMMs) and `bf16` (one product everywhere).
 
  (1) ON IDENTICAL, TRAINED WEIGHTS (each snapshot loaded into the CUDA path): total loss within 5e-4 relative, PSNR within
      0.01 dB, eikonal term within 1e-3 relative for bf16x3 / mixed (their forward passes are the same arithmetic; every
      rendered OUTPUT holds 1e-4 of its range, these are ratios of small differences of outputs), and the flat parameter gradient's
-     cosine similarity with the reference's autograd gradient >= 0.9999 (bf16x3) / >= 0.995 (mixed).  Deterministic.
- (2) TRAJECTORIES: training is chaotic - the four runs agree to < 1 % for ~75 steps, then decorrelate (any perturbation of
+     cosine similarity with the baseline's autograd gradient >= 0.9999 (bf16x3) / >= 0.995 (mixed).  Deterministic.
+ (2) TRAJECTORIES: training is chaotic - the runs agree to < 1 % for ~75 steps, then decorrelate (any perturbation of
      the order of fp32 rounding does that, the fp32 reference against itself included), so tail statistics are compared
-     within a band that reflects this: mean PSNR of the last 100 steps within 1.0 dB of the reference (observed spread over
-     repeated runs of this test: bf16x3 -0.6 .. -0.2 dB, mixed 0.0 .. +0.4 dB); loss and eikonal
+     within a band that reflects this: mean PSNR of the last 100 steps within 1.0 dB of the unmodified reference's stored
+     curve (observed spread over repeated runs of this test: bf16x3 -0.6 .. -0.2 dB, mixed 0.0 .. +0.4 dB); loss and eikonal
      tails are REPORTED (gpurun_out/precision_study.json -> profiles/), not asserted.
 `bf16` is reported only."""
 import json
 import os
 
+import numpy as np
 import pytest
 import torch
 
-from conftest import ROOT
+from conftest import GOLDEN, ROOT
+from oracle import neuconw_port as port
 from oracle import synth
 
 pytestmark = pytest.mark.gpu
@@ -78,30 +83,52 @@ def _ref_cfg():
                             n_outside=KW["n_outside"], n_vocab=KW["n_vocab"], perturb=0.0, cos_anneal_ratio=0.0, igr_weight=0.0001)
 
 
+def _initial_weights():
+    """the seeded initial weights of the CUDA path (TrainSystem seed), reference state_dict names"""
+    sysm = _make_nrw("bf16x3")
+    init = {k: v.detach().cpu().clone() for k, v in sysm.renderer.engine.named_params()}
+    init["embedding_a.weight"] = sysm.embedding_a.weight.detach().cpu().clone()
+    return init
+
+
+class _PortRunner:
+    """What oracle.ref_runner.RefRunner does with the reference's modules, on the restated step: render -> loss ->
+    backward -> clip_grad_norm_(0.99) -> Adam(eps=1e-7)."""
+
+    def __init__(self, cfg, init, device):
+        self.cfg = cfg
+        self.P = {k: v.to(device).clone() for k, v in init.items()}
+        self.optimizer = torch.optim.Adam(list(self.P.values()), lr=LR, eps=1e-7, weight_decay=0)
+
+    def train_step(self, batch):
+        res, loss, self.grads = port.train_step(self.P, self.cfg, batch, perturb_overwrite=0)
+        with torch.no_grad():
+            mse = ((res["color"].detach() - batch["rgbs"]) ** 2).mean()
+            self.last_metrics = {"loss": loss, "psnr": -10.0 * torch.log10(mse),
+                                 "eikonal": res["gradient_error"].detach().mean(), "s_val": res["s_val"].detach().mean()}
+        if self.optimizer is not None:
+            for k, p in self.P.items():
+                p.grad = self.grads[k]
+            torch.nn.utils.clip_grad_norm_(list(self.P.values()), 0.99)
+            self.optimizer.step()
+
+
 def _run_reference(init, batches, probe):
     """-> (curve, snapshots {step: (state dict, metrics on `probe`, flat-gradient dict on `probe`)})"""
-    from oracle import ref_runner
-
-    if not ref_runner.available():
-        pytest.skip("no reference copy on this box")
     cfg = _ref_cfg()
-    r = ref_runner.RefRunner(cfg, init, device="cuda", lr=LR)
+    r = _PortRunner(cfg, init, "cuda")
     hist, snaps = [], {}
     for i in range(STEPS):
         cfg.cos_anneal_ratio = min(1.0, i / 50000)                    # NeuconWSystem.get_cos_anneal_ratio
-        r.train_step(batches[i % len(batches)], perturb_overwrite=0)
+        r.train_step(batches[i % len(batches)])
         hist.append(torch.stack([r.last_metrics[k].reshape(()) for k in ("loss", "psnr", "eikonal", "s_val")]))
         if (i + 1) % 100 == 0:
-            state = {}
-            for pre, mod in (("neuconw.", r.m["neuconw"]), ("nerf.", r.m["nerf"]), ("embedding_a.", r.m["emb"])):
-                state.update({pre + k: v.detach().clone() for k, v in mod.state_dict().items()})
+            state = {k: v.detach().clone() for k, v in r.P.items()}
             opt, r.optimizer = r.optimizer, None                      # gradient only: no update on the probe batch
             cfg.cos_anneal_ratio = min(1.0, (i + 1) / 50000)
-            r.train_step(probe, perturb_overwrite=0)
+            r.train_step(probe)
             r.optimizer = opt
-            grads = {}
-            for pre, mod in (("neuconw.", r.m["neuconw"]), ("nerf.", r.m["nerf"])):
-                grads.update({pre + k: (p.grad.detach().clone() if p.grad is not None else torch.zeros_like(p)) for k, p in mod.named_parameters()})
+            grads = {k: g.detach().clone() for k, g in r.grads.items() if not k.startswith("embedding_a.")}
             snaps[i + 1] = (state, {k: float(v) for k, v in r.last_metrics.items()}, grads)
     return torch.stack(hist).cpu(), snaps
 
@@ -136,7 +163,8 @@ def test_precision_policy_training_curves():
     for mode in ("bf16x3", "mixed", "bf16"):
         curves[mode], init0 = _run_nrw(mode, batches)
         init = init or init0
-    curves["fp32_reference"], snaps = _run_reference(init, batches, probe)
+    curves["fp32_port"], snaps = _run_reference(init, batches, probe)
+    curves["fp32_reference"] = torch.from_numpy(np.load(os.path.join(GOLDEN, "precision_curve.npz"))["curve"])
     probes = {mode: _probe_nrw(mode, snaps, probe) for mode in ("bf16x3", "mixed", "bf16")}
     tail = {k: v[-100:].mean(0) for k, v in curves.items()}
     ref = tail["fp32_reference"]
@@ -148,9 +176,13 @@ def test_precision_policy_training_curves():
     os.makedirs(os.path.join(ROOT, "gpurun_out"), exist_ok=True)
     json.dump(report, open(os.path.join(ROOT, "gpurun_out", "precision_study.json"), "w"), indent=1)
     print(json.dumps({"tail": report["mean_of_last_100_steps"], "snapshots": probes}, indent=1))
-    # same starting point, and the baseline actually trains
-    assert abs(float(curves["bf16x3"][0, 0] - curves["fp32_reference"][0, 0])) < 1e-4 * abs(float(curves["fp32_reference"][0, 0]))
-    assert float(curves["fp32_reference"][-100:, 1].mean() - curves["fp32_reference"][:5, 1].mean()) > 10.0
+    # same starting point, the restated baseline follows the unmodified reference until the trajectories decorrelate,
+    # and the baseline actually trains
+    for mode in ("bf16x3", "fp32_port"):
+        assert abs(float(curves[mode][0, 0] - curves["fp32_reference"][0, 0])) < 1e-4 * abs(float(curves["fp32_reference"][0, 0])), mode
+    early = (curves["fp32_port"][:25, 0] - curves["fp32_reference"][:25, 0]).abs() / curves["fp32_reference"][:25, 0].abs()
+    assert float(early.max()) < 1e-2, float(early.max())
+    assert float(curves["fp32_port"][-100:, 1].mean() - curves["fp32_port"][:5, 1].mean()) > 10.0
     # (1) identical trained weights: forward quantities and gradient direction
     for mode, cos_min in (("bf16x3", 0.9999), ("mixed", 0.995)):
         for step, pr in probes[mode].items():

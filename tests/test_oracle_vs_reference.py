@@ -1,41 +1,45 @@
-"""Live comparison of the oracle port with the unmodified reference (build container only;
-skipped where /root/reference is absent, e.g. on the GPU box)."""
+"""Comparison of the oracle port with the unmodified reference on a configuration the CASES goldens do not cover
+(s_val_base 2, cos_anneal 0.25, 6 outside samples).  The reference's step on these inputs is stored in
+tests/golden/port_step.npz by oracle/make_golden.py: every output, the loss, a seeded sample of every parameter gradient
+with the gradient's max magnitude, and the state_dict layout of the reference's modules."""
+import json
+import os
+
 import numpy as np
 import pytest
-import torch
 
+from conftest import GOLDEN
 from oracle import neuconw_port as port
-from oracle import ref_import, synth
+from oracle import synth
+from oracle.make_golden import PORT_CFG, PORT_RAYS, PORT_SEED, sample_index
 
-pytestmark = pytest.mark.skipif(not ref_import.available(), reason="reference tree not present")
+
+@pytest.fixture(scope="module")
+def G():
+    return np.load(os.path.join(GOLDEN, "port_step.npz"))
 
 
-def test_port_vs_reference_live(params):
-    from oracle.make_golden import reference_train_step
-
-    cfg = synth.PathConfig(n_samples=12, n_importance=12, up_sample_steps=3, n_outside=6,
-                           s_val_base=2, cos_anneal_ratio=0.25, **synth.BRANDENBURG)
-    batch = synth.make_rays(24, cfg, seed=5)
-    res_r, loss_r, grads_r, _ = reference_train_step(cfg, params, batch, perturb_overwrite=0)
+def test_port_vs_reference_live(params, G):
+    cfg = synth.PathConfig(**PORT_CFG, **synth.BRANDENBURG)
+    batch = synth.make_rays(PORT_RAYS, cfg, seed=PORT_SEED)
     res_p, loss_p, grads_p = port.train_step(params, cfg, batch, perturb_overwrite=0)
-    assert abs(float(loss_r) - float(loss_p)) < 1e-5 * abs(float(loss_r))
-    for k in res_r:
-        a, b = res_p[k].detach().numpy(), res_r[k].detach().numpy()
+    loss_r = float(G["loss"])
+    assert abs(loss_r - float(loss_p)) < 1e-5 * abs(loss_r)
+    assert {k for k in G.files if k.startswith("out.")} == {"out." + k for k in res_p}
+    for k in res_p:
+        a, b = res_p[k].detach().numpy(), G["out." + k]
         assert a.shape == b.shape, k
         if a.size:
             assert np.abs(a - b).max() <= 1e-4 * (np.abs(b).max() + 1e-12), k
-    for k in grads_r:
-        a, b = grads_p[k].numpy(), grads_r[k].numpy()
-        assert np.abs(a - b).max() <= 1e-4 * (np.abs(b).max() + 1e-12), k
+    assert {k for k in G.files if k.startswith("gs.")} == {"gs." + k for k in grads_p}
+    for k, g in grads_p.items():
+        flat = g.reshape(-1)
+        a, b = flat[sample_index(flat.numel(), k)].numpy(), G["gs." + k]
+        assert np.abs(a - b).max() <= 1e-4 * (float(G["gmax." + k]) + 1e-12), k
+        assert abs(float(flat.abs().max()) - float(G["gmax." + k])) <= 1e-4 * (float(G["gmax." + k]) + 1e-12), k
 
 
-def test_state_dict_names_match_reference(params):
+def test_state_dict_names_match_reference(params, G):
     """oracle.synth parameter names/shapes == reference checkpoint layout (SURVEY.md §9.4)."""
-    from oracle.make_golden import build_reference
-
-    m = build_reference(synth.PathConfig(), params)
-    names = {}
-    for pre, mod in (("neuconw.", m["neuconw"]), ("nerf.", m["nerf"]), ("embedding_a.", m["emb"])):
-        for k, v in mod.state_dict().items():
-            names[pre + k] = tuple(v.shape)
+    names = {k: tuple(v) for k, v in json.loads(str(G["state_dict_layout"])).items()}
     assert names == {k: tuple(v.shape) for k, v in params.items()}
